@@ -151,16 +151,18 @@ struct Builder {
     const int ncols = gate ? 2 * N : N;
     int best = 0;
     long best_pad = -1;
-    for (int nc : {128, 96, 64, 32}) {
-      if (gate && nc % 64) continue;
-      if (!conv_tc_supported(K, nc, taps, dil)) continue;
-      const int per = gate ? nc / 2 : nc;
-      const long padded = long((N + per - 1) / per) * per;
-      if (best_pad < 0 || padded < best_pad) {
-        best_pad = padded;
-        best = nc;
+    // two M tiles per CTA; only when no width fits that, one (the default generator's K = 512 upsampler)
+    for (int m_tiles = 2; m_tiles >= 1 && !best; --m_tiles)
+      for (int nc : {128, 96, 64, 32}) {
+        if (gate && nc % 64) continue;
+        if (!conv_tc_supported(K, nc, taps, dil, m_tiles)) continue;
+        const int per = gate ? nc / 2 : nc;
+        const long padded = long((N + per - 1) / per) * per;
+        if (best_pad < 0 || padded < best_pad) {
+          best_pad = padded;
+          best = nc;
+        }
       }
-    }
     if (!best) return;
     const int NC = best, per = gate ? NC / 2 : NC;
     const int chunks = (N + per - 1) / per;
@@ -197,7 +199,8 @@ struct Builder {
   // Conv1d weight (Cout, Cin, k) -> [k][Cin][Cout]
   // tc: 0 = fp32 SIMT only, 1 = also pack for the tensor-core conv, 2 = gated (cout = 2 * channels),
   //     3 = token-level GEMM: fp16 hi/lo split packing (rowgemm_tc_kernel)
-  void conv(Lin& l, const std::string& base, int cout, int cin, int k, bool need_bias = true, int tc = 0) {
+  // dil: the dilation the tensor-core conv will run at (its shared-memory fit depends on it)
+  void conv(Lin& l, const std::string& base, int cout, int cin, int k, bool need_bias = true, int tc = 0, int dil = 1) {
     const OnnxTensor& w = hv.need(base + ".weight", {cout, cin, k});
     std::vector<float> t(size_t(k) * cin * cout);
     for (int o = 0; o < cout; ++o)
@@ -205,7 +208,7 @@ struct Builder {
         for (int j = 0; j < k; ++j) t[(size_t(j) * cin + i) * cout + o] = w.f32[(size_t(o) * cin + i) * k + j];
     if (tc == 3) rows_pack(l.rtc, t, k, cin, cout);
     else if (tc && cin % 16 == 0 && (tc == 2 ? (cout / 2) % 16 == 0 : cout % 4 == 0))
-      tc_pack(l.tc, t, k, cin, tc == 2 ? cout / 2 : cout, 1, tc == 2);
+      tc_pack(l.tc, t, k, cin, tc == 2 ? cout / 2 : cout, dil, tc == 2);
     place(&l.w, t);
     n_params += int64_t(t.size());
     l.cin = cin;
@@ -587,6 +590,18 @@ PackedVoice pack_voice(const HostVoice& hv) {
       B.place(&u.w, t);
       B.n_params += w.numel();
       B.vec(&u.b, "dec.ups." + std::to_string(i) + ".bias", u.cout);
+      // ResBlock1 stage on tensor cores: every conv of the stage is also packed for conv_tc_kernel, or none is
+      bool rb1_tc = c.resblock != "2" && nk >= 1 && nk <= 4;
+      if (rb1_tc) {
+        const int nd = int(c.rb_dils[0].size());
+        int ks[4] = {}, dl[4][3] = {};
+        for (int j = 0; j < nk; ++j) {
+          ks[j] = c.rb_kernels[j];
+          if (int(c.rb_dils[j].size()) != nd || nd > 3) rb1_tc = false;
+          for (int d = 0; d < nd && d < 3; ++d) dl[j][d] = c.rb_dils[j][d];
+        }
+        rb1_tc = rb1_tc && mrf1_tc_supported(u.cout, nk, nd, ks, dl);
+      }
       for (int j = 0; j < nk; ++j) {
         // NOTE: Builder records the address of every pointer slot, so the Lin objects must
         // already sit at their final address (pre-sized vectors, no copies afterwards).
@@ -600,8 +615,8 @@ PackedVoice pack_voice(const HostVoice& hv) {
           if (c.resblock == "2") {
             B.conv(rb.c1[d], rp + ".convs." + std::to_string(d), u.cout, u.cout, rb.k);
           } else {
-            B.conv(rb.c1[d], rp + ".convs1." + std::to_string(d), u.cout, u.cout, rb.k);
-            B.conv(rb.c2[d], rp + ".convs2." + std::to_string(d), u.cout, u.cout, rb.k);
+            B.conv(rb.c1[d], rp + ".convs1." + std::to_string(d), u.cout, u.cout, rb.k, true, rb1_tc ? 1 : 0, rb.dil[d]);
+            B.conv(rb.c2[d], rp + ".convs2." + std::to_string(d), u.cout, u.cout, rb.k, true, rb1_tc ? 1 : 0);
           }
         }
       }
@@ -1631,6 +1646,10 @@ Result* run_inference(Voice& v, const int64_t* ids, const int64_t* lengths, int 
     R.mark("upsample");
     Segs lvl{d_frm_off, d_frm_len, batch, Fmax};
     const MrfStageW& ms = dv.mrf[i];
+    bool rb1_tc = dv.use_tc;  // pack_voice packed every conv of a ResBlock1 stage for the tensor cores, or none
+    for (int j = 0; j < nk; ++j)
+      for (size_t d = 0; d < dv.rbs[i * nk + j].c1.size(); ++d)
+        rb1_tc = rb1_tc && !dv.rbs[i * nk + j].c2.empty() && dv.rbs[i * nk + j].c1[d].tc.ok && dv.rbs[i * nk + j].c2[d].tc.ok;
     if (dv.use_tc && ms.ok) {
       MrfParams mp;
       mp.x = xu;
@@ -1659,6 +1678,32 @@ Result* run_inference(Voice& v, const int64_t* ids, const int64_t* lengths, int 
       if (!v1 && mrf_ws_supported(mp, u.cout)) launch_mrf_ws(mp, dv.tc_fmt, batch, Fmax, st);
       else if (!v1 && mrf_ws128_supported(mp, u.cout)) launch_mrf_ws128(mp, dv.tc_fmt, batch, Fmax, st);
       else launch_mrf_tc(mp, u.cout, dv.tc_fmt, batch, Fmax, st);
+    } else if (rb1_tc) {
+      // ResBlock1 on tensor cores: one conv_tc_kernel per conv, the residual add and the 1/nk mean in the second
+      // conv's epilogue; same buffers as the fp32 branch below
+      for (int j = 0; j < nk; ++j) {
+        const ResBlockW& rb = dv.rbs[i * nk + j];
+        const float* src = xu;
+        const size_t nd = rb.dil.size();
+        for (size_t d = 0; d < nd; ++d) {
+          const bool last = d + 1 == nd;
+          // t = conv1_d(lrelu(x)) + b1; x = x + conv2_d(lrelu(t)) + b2 (each conv reads rows outside the utterance as 0)
+          TcConvParams p = R.base_tc(rb.c1[d].tc, rb.c1[d].b, src, u.cout, tb, u.cout, lvl, out_scale);
+          p.dil = rb.dil[d];
+          p.in_slope = 0.1f;
+          R.tc_conv(p, lvl);
+          TcConvParams q = R.base_tc(rb.c2[d].tc, rb.c2[d].b, tb, u.cout, last ? sum : yb[d & 1], u.cout, lvl, out_scale);
+          q.in_slope = 0.1f;
+          q.res = src;
+          q.res_stride = u.cout;
+          if (last) {
+            q.scale = 1.0f / float(nk);
+            q.accumulate = j == 0 ? 0 : 1;
+          }
+          launch_conv_tc_res(q, dv.tc_fmt, lvl.n, lvl.max_len, st);
+          src = yb[d & 1];
+        }
+      }
     } else
     for (int j = 0; j < nk; ++j) {
       const ResBlockW& rb = dv.rbs[i * nk + j];

@@ -113,9 +113,24 @@ struct TcConvParams {
   int in_scale = 1, out_scale = 1, rows_extra = 0;
   int ups_u = 1, ups_pad = 0, ups_cout = 0;
   int wide = 0;  // 256-bit global stores in the polyphase epilogue (set by the launcher: M3B200_WIDE_IO + alignment)
+  // residual epilogue (launch_conv_tc_res only): o = (acc + bias + res) * scale; out = accumulate ? out + o : o
+  const float* res = nullptr;
+  int res_stride = 0;
+  float scale = 1.f;
+  int accumulate = 0;
 };
-bool conv_tc_supported(int K, int NC, int taps, int dil);
+// m_tiles: 128-row M tiles per CTA, 2 or 1.  launch_conv_tc runs 2 whenever they fit shared memory and 1 otherwise,
+// so a weight packing accepted for 1 tile only (K = 512 with 2 taps, the default generator's first upsampler) runs too.
+bool conv_tc_supported(int K, int NC, int taps, int dil, int m_tiles = 2);
 void launch_conv_tc(const TcConvParams& p, int fmt, int n_seg, int max_seg_len, cudaStream_t st);
+// conv_tc_kernel with the residual epilogue above: the second conv of a ResBlock1 dilation step
+// (x = x + conv2(lrelu(t)) + b2), and for the last step the 1/nk mean into the stage sum.
+void launch_conv_tc_res(const TcConvParams& p, int fmt, int n_seg, int max_seg_len, cudaStream_t st);
+// Every conv of a ResBlock1 MRF stage (C channels, nk resblocks of nd dilations, kernel sizes k[j], dilations dil[j][d])
+// fits conv_tc_kernel with two M tiles: C % 32 == 0, nk <= 4, nd <= 3, odd k <= 11, and the A operand of
+// 256 + (k-1)*dil rows x C channels plus two weight stages within 225 KB of shared memory.  That holds for every
+// k <= 11, dil <= 5 up to C = 288; C = 320 / 352 fit only up to (k-1)*dil = 39 / 7, and C >= 384 never fits.
+bool mrf1_tc_supported(int C, int nk, int nd, const int* k, const int (*dil)[3]);
 // kernels_tc_ups.cu: the TC_UPS case with a shared-memory bias and an early accumulator release; the default
 // for the polyphase upsamplers since round 2 (bit-identical to conv_tc_kernel's TC_UPS epilogue, which
 // M3B200_UPS_V1=1 selects again).

@@ -22,13 +22,15 @@
 
 namespace m3 {
 
-constexpr int CT_NT = 2;           // M tiles per CTA
-constexpr int CT_R = CT_NT * 128;  // rows per CTA
+constexpr int CT_NT = 2;  // M tiles per CTA (1 for shapes whose A operand only fits shared memory at 128 rows)
 constexpr int CT_THREADS = 320;
 constexpr int CT_SMEM_MAX = 225 * 1024;
 
-template <int FMT>
+// RES: residual epilogue of launch_conv_tc_res (p.epi is ignored); NT: M tiles (128 rows each) per CTA.  Template
+// arguments, so that the instantiation every other caller runs (RES = false, NT = 2) compiles exactly as without them.
+template <int FMT, bool RES, int NT>
 __global__ void __launch_bounds__(CT_THREADS, 1) conv_tc_kernel(TcConvParams p, int stages, int rows_a) {
+  constexpr int CT_R = NT * 128;  // rows per CTA
   using E = tc::Elem<FMT>;
   extern __shared__ __align__(128) uint8_t smem[];
   __shared__ uint32_t tmem_slot;
@@ -141,11 +143,11 @@ __global__ void __launch_bounds__(CT_THREADS, 1) conv_tc_kernel(TcConvParams p, 
           for (int ks = 0; ks < p.K / 16; ++ks) {
             const uint64_t bd = tc::make_desc(wbase + uint32_t(ks * 2 * NC) * 16u, uint32_t(NC) * 16u, 128u);
 #pragma unroll
-            for (int m = 0; m < CT_NT; ++m) {
+            for (int m = 0; m < NT; ++m) {
               const int arow = m * 128 + tap * p.dil;
               const uint64_t ad =
                   tc::make_desc(abase + uint32_t((ks * 2) * rows_a + arow) * 16u, uint32_t(rows_a) * 16u, 128u);
-              tc::mma_f16_ss(tmem + uint32_t(b * CT_NT + m) * NC, ad, bd, idesc, (tap | ks) ? 1u : 0u);
+              tc::mma_f16_ss(tmem + uint32_t(b * NT + m) * NC, ad, bd, idesc, (tap | ks) ? 1u : 0u);
             }
           }
           tc::mma_commit(&empty_bar[s]);
@@ -162,11 +164,11 @@ __global__ void __launch_bounds__(CT_THREADS, 1) conv_tc_kernel(TcConvParams p, 
       const int b = c & 1;
       tc::mbar_wait(&acc_full[b], ((c >> 1) & 1));
       tc::fence_after_sync();
-      for (int m = 0; m < CT_NT; ++m) {
+      for (int m = 0; m < NT; ++m) {
         const int t = t0 + m * 128 + q * 32 + lane;
         const bool row_ok = t < rows;
-        const uint32_t acc = lane_base + uint32_t(b * CT_NT + m) * NC;
-        if (p.epi == TC_GATE) {
+        const uint32_t acc = lane_base + uint32_t(b * NT + m) * NC;
+        if (!RES && p.epi == TC_GATE) {
           const int cpt = NC / 4;  // gated channels per thread
           for (int cc = 0; cc < cpt; cc += 16) {
             __syncwarp();
@@ -213,6 +215,36 @@ __global__ void __launch_bounds__(CT_THREADS, 1) conv_tc_kernel(TcConvParams p, 
             tc::tmem_ld_wait();
             if (!row_ok) continue;
             const int n0 = c * NC + j0;
+            if constexpr (RES) {
+              // same operation order as the fp32 conv's epilogue: ((acc + bias) + res) * scale, then store or add
+              if (t >= out_len) continue;
+              const long long orow = out_base + t;
+              float4 r[4], cur[4];
+#pragma unroll
+              for (int e4 = 0; e4 < 4; ++e4) {  // all operands in flight together
+                const int n = n0 + e4 * 4;
+                if (n >= p.N) continue;
+                r[e4] = *reinterpret_cast<const float4*>(p.res + orow * p.res_stride + n);
+                if (p.accumulate) cur[e4] = *reinterpret_cast<const float4*>(p.out + orow * p.out_stride + p.out_coff + n);
+              }
+#pragma unroll
+              for (int e4 = 0; e4 < 4; ++e4) {
+                const int n = n0 + e4 * 4;
+                if (n >= p.N) continue;
+                const float* rr = reinterpret_cast<const float*>(&r[e4]);
+                float o[4];
+#pragma unroll
+                for (int f = 0; f < 4; ++f) o[f] = (v[e4 * 4 + f] + p.bias[n + f] + rr[f]) * p.scale;
+                if (p.accumulate) {
+                  o[0] += cur[e4].x;
+                  o[1] += cur[e4].y;
+                  o[2] += cur[e4].z;
+                  o[3] += cur[e4].w;
+                }
+                *reinterpret_cast<float4*>(p.out + orow * p.out_stride + p.out_coff + n) = make_float4(o[0], o[1], o[2], o[3]);
+              }
+              continue;
+            }
             if (p.epi == TC_UPS && p.wide) {
               // same mapping, one full 32-byte sector per lane and store (Cout % 8 == 0: the 8 columns of a
               // group share their phase)
@@ -292,35 +324,72 @@ __global__ void __launch_bounds__(CT_THREADS, 1) conv_tc_kernel(TcConvParams p, 
   if (warp == 0) tc::tmem_dealloc<512>(tmem);
 }
 
-bool conv_tc_supported(int K, int NC, int taps, int dil) {
+bool conv_tc_supported(int K, int NC, int taps, int dil, int m_tiles) {
   if (K % 16 || K < 16 || K > 512) return false;
   if (NC % 32 || NC < 32 || NC > 128) return false;  // 2 buffers x 2 tiles x NC <= 512 TMEM columns
-  const size_t a_bytes = size_t(K / 8) * ((CT_R + (taps - 1) * dil) | 1) * 16 + 128;
+  if (m_tiles != 1 && m_tiles != CT_NT) return false;
+  const size_t a_bytes = size_t(K / 8) * ((m_tiles * 128 + (taps - 1) * dil) | 1) * 16 + 128;
   const size_t stage = size_t(K) * NC * 2;
   return a_bytes + 2 * stage <= size_t(CT_SMEM_MAX);
 }
 
-void launch_conv_tc(const TcConvParams& p_in, int fmt, int n_seg, int max_seg_len, cudaStream_t st) {
+bool mrf1_tc_supported(int C, int nk, int nd, const int* k, const int (*dil)[3]) {
+  if (C % 32 || nk < 1 || nk > 4 || nd < 1 || nd > 3) return false;
+  for (int j = 0; j < nk; ++j) {
+    if (k[j] < 1 || k[j] > 11 || !(k[j] & 1)) return false;
+    for (int d = 0; d < nd; ++d) {
+      if (dil[j][d] < 1) return false;
+      if (!conv_tc_supported(C, 32, k[j], dil[j][d])) return false;  // NC = 32 is the smallest packing
+    }
+  }
+  return true;
+}
+
+template <bool RES, int NT>
+static void launch_nt(const TcConvParams& p, int fmt, dim3 grid, size_t smem, int stages, int rows_a, cudaStream_t st) {
+  ensure_max_dynamic_smem(fmt ? reinterpret_cast<const void*>(conv_tc_kernel<1, RES, NT>)
+                              : reinterpret_cast<const void*>(conv_tc_kernel<0, RES, NT>));
+  if (fmt) conv_tc_kernel<1, RES, NT><<<grid, CT_THREADS, smem, st>>>(p, stages, rows_a);
+  else conv_tc_kernel<0, RES, NT><<<grid, CT_THREADS, smem, st>>>(p, stages, rows_a);
+}
+
+template <bool RES>
+static void launch_conv_tc_impl(const TcConvParams& p_in, int fmt, int n_seg, int max_seg_len, cudaStream_t st) {
   TcConvParams p = p_in;
-  p.wide = (p.epi == TC_UPS && wide_io_enabled() && p.ups_cout % 8 == 0 && p.out_stride % 8 == 0 &&
+  p.wide = (!RES && p.epi == TC_UPS && wide_io_enabled() && p.ups_cout % 8 == 0 && p.out_stride % 8 == 0 &&
             (reinterpret_cast<uintptr_t>(p.out) & 31u) == 0)
                ? 1
                : 0;
   const int rows = max_seg_len * p.in_scale + p.rows_extra;
   if (rows <= 0 || n_seg <= 0) return;
-  const int rows_a = (CT_R + (p.taps - 1) * p.dil) | 1;  // odd row pitch: conflict-free chunk-major smem stores
-  const size_t a_bytes = (size_t(p.K / 8) * rows_a * 16 + 127) & ~size_t(127);
+  // two M tiles per CTA whenever two weight stages fit next to the A operand, else one (e.g. K = 512 polyphase upsampler)
+  int nt = CT_NT, rows_a = 0, stages = 0;
+  size_t a_bytes = 0;
   const size_t stage = size_t(p.K) * p.NC * 2;
-  int stages = int((size_t(CT_SMEM_MAX) - a_bytes) / stage);
-  stages = std::min(4, stages);
-  if (stages < 2) throw std::runtime_error("conv_tc: shape does not fit shared memory");
+  for (; nt >= 1; --nt) {
+    rows_a = (nt * 128 + (p.taps - 1) * p.dil) | 1;  // odd row pitch: conflict-free chunk-major smem stores
+    a_bytes = (size_t(p.K / 8) * rows_a * 16 + 127) & ~size_t(127);
+    stages = a_bytes < size_t(CT_SMEM_MAX) ? std::min(4, int((size_t(CT_SMEM_MAX) - a_bytes) / stage)) : 0;
+    if (stages >= 2) break;
+  }
+  if (nt < 1) throw std::runtime_error("conv_tc: shape does not fit shared memory");
   // >= 120 KB keeps a single CTA per SM (each CTA owns all 512 TMEM columns)
   const size_t smem = std::max(a_bytes + stages * stage, size_t(120 * 1024));
-  dim3 grid((rows + CT_R - 1) / CT_R, n_seg);
-  ensure_max_dynamic_smem(fmt ? reinterpret_cast<const void*>(conv_tc_kernel<1>) : reinterpret_cast<const void*>(conv_tc_kernel<0>));
-  if (fmt) conv_tc_kernel<1><<<grid, CT_THREADS, smem, st>>>(p, stages, rows_a);
-  else conv_tc_kernel<0><<<grid, CT_THREADS, smem, st>>>(p, stages, rows_a);
-  post_launch("conv_tc_kernel", st);
+  const int R = nt * 128;
+  dim3 grid((rows + R - 1) / R, n_seg);
+  if (nt == CT_NT) launch_nt<RES, CT_NT>(p, fmt, grid, smem, stages, rows_a, st);
+  else launch_nt<RES, 1>(p, fmt, grid, smem, stages, rows_a, st);
+  post_launch(RES ? "conv_tc_kernel(res)" : "conv_tc_kernel", st);
+}
+
+void launch_conv_tc(const TcConvParams& p, int fmt, int n_seg, int max_seg_len, cudaStream_t st) {
+  launch_conv_tc_impl<false>(p, fmt, n_seg, max_seg_len, st);
+}
+
+void launch_conv_tc_res(const TcConvParams& p, int fmt, int n_seg, int max_seg_len, cudaStream_t st) {
+  if (!p.res || !p.bias || p.N % 16 || p.res_stride % 4 || p.out_stride % 4 || p.out_coff % 4)
+    throw std::runtime_error("conv_tc_res: needs res and bias, N % 16 == 0 and 16-byte aligned rows");
+  launch_conv_tc_impl<true>(p, fmt, n_seg, max_seg_len, st);
 }
 
 }  // namespace m3

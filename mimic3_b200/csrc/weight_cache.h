@@ -20,7 +20,7 @@
 
 namespace m3 {
 
-constexpr uint32_t kCacheLayoutVersion = 9;  // bump whenever pack_voice's output or a *W struct changes
+constexpr uint32_t kCacheLayoutVersion = 10;  // bump whenever pack_voice's output or a *W struct changes
 
 struct CacheKey {
   std::string onnx_path, config_path;  // resolved

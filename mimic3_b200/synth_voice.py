@@ -64,6 +64,23 @@ def low_config(n_speakers: int = 1, num_symbols: int = 50) -> SynthModelConfig:
     )
 
 
+def default_config(n_speakers: int = 1, num_symbols: int = 50) -> SynthModelConfig:
+    """Generator of the reference ``ModelConfig`` defaults (``mimic3_tts/config.py:126-135``):
+    ResBlock1, 512 initial channels, upsampling 8*8*2*2 -- what a voice gets when its
+    training config leaves the generator section alone."""
+    return SynthModelConfig(
+        num_symbols=num_symbols,
+        n_speakers=n_speakers,
+        resblock="1",
+        resblock_kernel_sizes=(3, 7, 11),
+        resblock_dilation_sizes=((1, 3, 5), (1, 3, 5), (1, 3, 5)),
+        upsample_rates=(8, 8, 2, 2),
+        upsample_initial_channel=512,
+        upsample_kernel_sizes=(16, 16, 4, 4),
+        gin_channels=512 if n_speakers > 1 else 0,
+    )
+
+
 def tiny_config(n_speakers: int = 1, num_symbols: int = 20, resblock: str = "2",
                 use_sdp: bool = True) -> SynthModelConfig:
     """Small shapes for fast CPU/GPU tests; same graph, same code paths."""

@@ -1,7 +1,8 @@
 """One small invocation of the whole hot path on the `_low`-shaped voice (so every fused tensor-core kernel launches),
 meant to run under compute-sanitizer:
-    compute-sanitizer --tool memcheck|racecheck|synccheck python tools/sanitize_run.py
-No oracle, no timing; two short ragged utterances, voice-default noise scales."""
+    compute-sanitizer --tool memcheck|racecheck|synccheck python tools/sanitize_run.py [--default]
+No oracle, no timing; three short ragged utterances, voice-default noise scales.  --default: the ResBlock1 generator
+of the reference ModelConfig defaults (synth_voice.default_config) instead."""
 import sys
 import tempfile
 from pathlib import Path
@@ -18,7 +19,8 @@ from mimic3_b200.engine import B200Session  # noqa: E402
 def main():
     with tempfile.TemporaryDirectory() as d:
         vd = Path(d) / "voice"
-        sv.write_voice(vd, sv.low_config(n_speakers=3), seed=5)
+        cfg = sv.default_config(n_speakers=3) if "--default" in sys.argv[1:] else sv.low_config(n_speakers=3)
+        sv.write_voice(vd, cfg, seed=5)
         sess = B200Session(str(vd), device=0)
         rng = np.random.default_rng(1)
         lengths = np.array([23, 9, 14], dtype=np.int64)
