@@ -259,39 +259,106 @@ class VitsOracle:
         return z
 
     # ---- A.4 HiFi-GAN --------------------------------------------------------------
-    def decoder(self, z, g, taps=None):
-        m = self.m
-        x = self.conv(z, "dec.conv_pre", padding=3)
+    # The generator is split into a pre-stage (conv_pre + speaker cond), one stage per upsampler (ConvTranspose1d
+    # + MRF) and a post-stage (conv_post + tanh), so that a test can feed each stage the engine's own input.
+    #
+    # Each piece runs in the dtype of its input: float32 is the oracle itself, float64 a high-precision reference.
+    # ``rounding`` maps a conv group -- "pre", f"ups{i}", f"mrf{i}", "post" -- to "fp16" or "bf16": the input of
+    # every conv in that group (after its leaky-relu) and its float32 weights are rounded to that format before
+    # the product, which is what the engine's tensor-core kernels stage.  Biases, residual adds and the
+    # accumulation stay in the input dtype.  Groups not in ``rounding`` are not rounded.
+    _RND = {"fp16": torch.float16, "bf16": torch.bfloat16}
+
+    def _gconv(self, x, name, fmt, transpose=False, bias=True, **kw):
+        """One generator conv in x's dtype; ``fmt`` rounds its operands (see above)."""
+        w = self.P[name + ".weight"]
+        b = self.P.get(name + ".bias") if bias else None
+        if fmt is not None:
+            x = x.to(self._RND[fmt]).to(x.dtype)
+            w = w.to(self._RND[fmt])
+        w = w.to(x.dtype)
+        if b is not None:
+            b = b.to(x.dtype)
+        return self._conv1d(x, w, b, name, transpose, **kw)
+
+    def _conv1d(self, x, w, b, name, transpose, **kw):
+        """The single place every generator conv goes through (tests override it to inject defects)."""
+        return (F.conv_transpose1d if transpose else F.conv1d)(x, w, b, **kw)
+
+    def decoder_pre(self, z, g, rounding=None):
+        x = self._gconv(z, "dec.conv_pre", (rounding or {}).get("pre"), padding=3)
         if g is not None:
-            x = x + self.conv(g, "dec.cond")
+            x = x + self._gconv(g.to(z.dtype), "dec.cond", None)
+        return x
+
+    def decoder_stage(self, i, x, rounding=None):
+        """Upsampler i, then its multi-receptive-field fusion (the mean of nk resblocks)."""
+        m = self.m
+        rounding = rounding or {}
+        u, k = m["upsample_rates"][i], m["upsample_kernel_sizes"][i]
+        fu, fm = rounding.get(f"ups{i}"), rounding.get(f"mrf{i}")
         nk = len(m["resblock_kernel_sizes"])
-        for i, (u, k) in enumerate(zip(m["upsample_rates"], m["upsample_kernel_sizes"])):
-            x = F.leaky_relu(x, LRELU_SLOPE)
-            x = F.conv_transpose1d(x, self.P[f"dec.ups.{i}.weight"], self.P[f"dec.ups.{i}.bias"],
-                                   stride=u, padding=(k - u) // 2)
-            xs = None
-            for j, (rk, dils) in enumerate(zip(m["resblock_kernel_sizes"], m["resblock_dilation_sizes"])):
-                rb = f"dec.resblocks.{i * nk + j}"
-                y = x
-                for d_i, d in enumerate(dils):
-                    if str(m["resblock"]) == "2":
-                        t = self.conv(F.leaky_relu(y, LRELU_SLOPE), f"{rb}.convs.{d_i}",
-                                      dilation=d, padding=d * (rk - 1) // 2)
-                    else:
-                        t = self.conv(F.leaky_relu(y, LRELU_SLOPE), f"{rb}.convs1.{d_i}",
-                                      dilation=d, padding=d * (rk - 1) // 2)
-                        t = self.conv(F.leaky_relu(t, LRELU_SLOPE), f"{rb}.convs2.{d_i}",
-                                      dilation=1, padding=(rk - 1) // 2)
-                    y = y + t
-                xs = y if xs is None else xs + y
-            x = xs / nk
-            if taps is not None:
-                taps[f"mrf{i}"] = x[0].t().numpy().copy()
+        x = F.leaky_relu(x, LRELU_SLOPE)
+        x = self._gconv(x, f"dec.ups.{i}", fu, transpose=True, stride=u, padding=(k - u) // 2)
+        xs = None
+        for j, (rk, dils) in enumerate(zip(m["resblock_kernel_sizes"], m["resblock_dilation_sizes"])):
+            rb = f"dec.resblocks.{i * nk + j}"
+            y = x
+            for d_i, d in enumerate(dils):
+                if str(m["resblock"]) == "2":
+                    t = self._gconv(F.leaky_relu(y, LRELU_SLOPE), f"{rb}.convs.{d_i}", fm,
+                                    dilation=d, padding=d * (rk - 1) // 2)
+                else:
+                    t = self._gconv(F.leaky_relu(y, LRELU_SLOPE), f"{rb}.convs1.{d_i}", fm,
+                                    dilation=d, padding=d * (rk - 1) // 2)
+                    t = self._gconv(F.leaky_relu(t, LRELU_SLOPE), f"{rb}.convs2.{d_i}", fm,
+                                    dilation=1, padding=(rk - 1) // 2)
+                y = y + t
+            xs = y if xs is None else xs + y
+        return xs / nk
+
+    def decoder_post(self, x, rounding=None):
         x = F.leaky_relu(x)  # slope 0.01
-        x = F.conv1d(x, self.P["dec.conv_post.weight"], None, padding=3)
+        x = self._gconv(x, "dec.conv_post", (rounding or {}).get("post"), bias=False, padding=3)
         return torch.tanh(x)
 
+    def decoder(self, z, g, taps=None):
+        x = self.decoder_pre(z, g)
+        for i in range(len(self.m["upsample_rates"])):
+            x = self.decoder_stage(i, x)
+            if taps is not None:
+                taps[f"mrf{i}"] = x[0].t().numpy().copy()
+        return self.decoder_post(x)
+
     # ---- A.0 top level ---------------------------------------------------------------
+    def _front(self, ids, noise_w, length_scale, sid, seed, row):
+        """Text encoder, speaker embedding and duration predictor: everything before the length regulator."""
+        T = int(ids.shape[0])
+        x, m_p, logs_p = self.text_encoder(ids)
+        g = self.speaker(sid)
+        if self.use_sdp:
+            zn = torch.zeros(1, 2, T)
+            if noise_w != 0:
+                zn = torch.from_numpy(philox.normal(seed, 0, row, np.arange(T)[None, :], np.arange(2)[:, None]))[None]
+            logw = self.sdp(x, g, float(noise_w), zn)
+        else:
+            logw = self.dp_plain(x, g)
+        w = torch.exp(logw) * float(length_scale)
+        dur = torch.ceil(w)[0, 0].to(torch.int64)
+        return x, m_p, logs_p, g, logw, dur
+
+    @torch.no_grad()
+    def durations(self, ids, scales=None, sid: Optional[int] = None, seed: int = 0, row: int = 0) -> np.ndarray:
+        """Integer frames per id, as ``infer`` computes them, without the flow and the decoder; the utterance has
+        ``max(1, durations.sum())`` frames."""
+        _, length_scale, noise_w = scales if scales is not None else self.defaults
+        ids = torch.as_tensor(np.asarray(ids, dtype=np.int64))
+        return self._front(ids, noise_w, length_scale, sid, seed, row)[5].numpy()
+
+    def speaker(self, sid: Optional[int]):
+        """The speaker embedding g (1, G, 1) the decoder's cond conv reads; None for single-speaker voices."""
+        return self.P["emb_g.weight"][int(sid or 0)][None, :, None] if self.multispeaker else None
+
     @torch.no_grad()
     def infer(self, ids, scales=None, sid: Optional[int] = None, seed: int = 0, row: int = 0,
               return_intermediates: bool = False):
@@ -303,20 +370,7 @@ class VitsOracle:
         ids = torch.as_tensor(np.asarray(ids, dtype=np.int64))
         T = int(ids.shape[0])
         inter: Dict[str, np.ndarray] = {}
-        x, m_p, logs_p = self.text_encoder(ids)
-        g = None
-        if self.multispeaker:
-            g = self.P["emb_g.weight"][int(sid or 0)][None, :, None]
-        if self.use_sdp:
-            zn = torch.zeros(1, 2, T)
-            if noise_w != 0:
-                zn = torch.from_numpy(philox.normal(seed, 0, row, np.arange(T)[None, :], np.arange(2)[:, None]))[None]
-            logw = self.sdp(x, g, float(noise_w), zn)
-        else:
-            logw = self.dp_plain(x, g)
-        w = torch.exp(logw) * float(length_scale)
-        w_ceil = torch.ceil(w)[0, 0]
-        dur = w_ceil.to(torch.int64)
+        x, m_p, logs_p, g, logw, dur = self._front(ids, noise_w, length_scale, sid, seed, row)
         Fr = max(1, int(dur.sum()))
         cum = torch.cumsum(dur, 0)
         tok = torch.searchsorted(cum, torch.arange(Fr), right=True)  # frame -> token (cum[t-1] <= y < cum[t])
